@@ -2,6 +2,7 @@
 """bench.py - 48 kHz samples/s through encode -> quantize -> lookup -> decode (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload symad|v1|v1_bf16|stream_v1]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -24,6 +25,9 @@ NCCL is used only for the timing barrier and the max-over-ranks of the device ti
                the host cores - one process and all cores - and, informational, as eager PyTorch on this GPU.
 `--impl reference`: the reference's own CPU implementation of the path.  The reference is pure Python on
                torch CPU ops and cannot travel to the GPU box, so this leg times the oracle port on all host cores.
+`--dump-outputs DIR`: after the timed steps, what the last of them returned to its caller - the decoded waveforms and the
+               code indices of rank 0's batch - as DIR/waveform.npy and DIR/indices.npy.  Inputs are seeded, so two builds
+               run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -382,7 +386,7 @@ def run_ours(args):
     x_dev = [x.to(dev) for x in x_host]
 
     def step(i):
-        return codec_step(tx, rx, dec, x_dev[i % n_in])[0]
+        return codec_step(tx, rx, dec, x_dev[i % n_in])
 
     def barrier():
         if world > 1:
@@ -409,26 +413,31 @@ def run_ours(args):
         torch.cuda.synchronize(dev)
     for i in range(args.warmup):
         step(i)
-    # The timed region - EXACTLY K steps between barrier + synchronize on both sides, device time by CUDA events, max over ranks - is
-    # measured `--regions` R times back to back and the MEDIAN region is reported (all R values are on the line as
-    # `timed_regions_ms_per_step`).  Reason: on these power-capped boxes (sw_power_cap at ~1 kW) about one region in four runs 15-60 %
-    # slow for its ~100 ms (three of twelve single-region runs of the same build in round 2: 10.0 .. 10.3 ms vs 11.8 / 15.2 / 16.0),
-    # while the e2e loop and the per-launch event sums of the same process stay put; a single region is a coin flip, the median is not.
+    # The K timed steps run as R = min(--regions, K) back-to-back regions (K split as evenly as possible), each between barrier +
+    # synchronize on both sides, device time by CUDA events, max over ranks; the MEDIAN region's time per step is reported (every
+    # region is on the line as `timed_regions_ms_per_step`).  Reason: on power-capped B200 boxes (sw_power_cap at ~1 kW) about one
+    # 100 ms region in four ran 15-60 % slow (three of twelve single-region runs of the same build: 10.0 .. 10.3 ms vs 11.8 / 15.2 /
+    # 16.0), while the e2e loop and the per-launch event sums of the same process stayed put; one region is a coin flip, the median is not.
+    n_regions = max(1, min(args.regions, args.steps))
+    region_steps = [args.steps // n_regions + (r < args.steps % n_regions) for r in range(n_regions)]
     regions = []
-    for r in range(max(1, args.regions)):
-        l0 = tx.launch_count + rx.launch_count + dec.launch_count
+    l0 = tx.launch_count + rx.launch_count + dec.launch_count
+    i = 0
+    for n in region_steps:
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         w0 = time.time()
         e0.record()
-        for i in range(args.steps):
-            y = step(i)
+        for _ in range(n):
+            y, idx = step(i)
+            i += 1
         e1.record()
         barrier()
         w1 = time.time()
-        regions.append((max_over_ranks(e0.elapsed_time(e1)), w0, w1))
+        regions.append((max_over_ranks(e0.elapsed_time(e1)) / n, w0, w1))
     order = sorted(range(len(regions)), key=lambda k: regions[k][0])
-    ms_total, w0, w1 = regions[order[(len(regions) - 1) // 2]]
+    ms_step, w0, w1 = regions[order[(len(regions) - 1) // 2]]
+    launches = tx.launch_count + rx.launch_count + dec.launch_count - l0
     clocks = sampler.stop(w0, w1) if rank == 0 else None
     if os.environ.get("ADEC_BENCH_DEBUG") and rank == 0:
         # diagnostic: the same K steps with a device synchronise after each (does sustained back-to-back load run slower on this box?)
@@ -439,8 +448,7 @@ def run_ours(args):
             a0.record(); step(i); a1.record()
             torch.cuda.synchronize(dev)
             per.append(a0.elapsed_time(a1))
-        print(f"synced per-step ms: {[round(v, 3) for v in per]}; back-to-back mean {ms_total / args.steps:.3f}", file=sys.stderr)
-    launches = (tx.launch_count + rx.launch_count + dec.launch_count - l0)
+        print(f"synced per-step ms: {[round(v, 3) for v in per]}; back-to-back median region {ms_step:.3f}", file=sys.stderr)
     dbg_run = any(k.startswith("ADEC_DBG_") for k in os.environ)    # timing experiments with deliberately wrong results (tools/gpu_dbg.sh)
     assert dbg_run or torch.isfinite(y).all()
     if not dbg_run and (tx.range_error() or dec.range_error()):
@@ -482,8 +490,8 @@ def run_ours(args):
                 print(f"  {k:44s} {v[1] / v[0]:8.3f} ms  {v[2] / (v[1] / v[0]) / 1e6:8.1f} GB/s(alg)", file=sys.stderr)
             print(f"  sum of launches per step: {tot / 2:.3f} ms", file=sys.stderr)
         dname, (dn, dms, dbytes) = top[0]
-        step_ms = ms_total / args.steps                 # shares are of the TIMED step (which also holds the RVQ / lookup launches)
-        prof = {"kernel": dname, "launch_ms": dms / dn, "alg_bytes_per_launch": dbytes, "share_of_step": (dms / dn) / step_ms,
+        # shares are of the TIMED step (which also holds the RVQ / lookup launches)
+        prof = {"kernel": dname, "launch_ms": dms / dn, "alg_bytes_per_launch": dbytes, "share_of_step": (dms / dn) / ms_step,
                 "conv_launches_ms_per_step": tot / 2,
                 "top5": [{"op": k, "ms": v[1] / v[0], "GBps": v[2] / (v[1] / v[0]) / 1e6} for k, v in top[:5]]}
 
@@ -491,8 +499,17 @@ def run_ours(args):
         dist.destroy_process_group()
     if rank != 0:
         return
+    if args.dump_outputs:
+        # What a caller of the timed path received in the last timed step (rank 0's shard: the inputs of a one-GPU run), at most
+        # 26 MB (v1_bf16).  It is the same from run to run: a step's output depends on the inputs of at most the last 16 steps (one
+        # step for 1 s utterances), and those are seeded and fixed - the 1.5 s pre-warm loop repeats step 0 more than 16 times in
+        # every workload.
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "waveform.npy"), y.cpu().numpy())                        # (B,1,T) float32
+        np.save(os.path.join(args.dump_outputs, "indices.npy"), idx.cpu().numpy().astype(np.float64))   # (Nq,B,F), exact
     samples_per_step = world * B * T
-    value = samples_per_step * args.steps / (ms_total / 1e3)
+    value = samples_per_step / (ms_step / 1e3)
     e2e_value = samples_per_step * args.steps / (ms_e2e / 1e3)
     peak, peak_src, peaks = measured_peaks()
     per_gpu = value / world
@@ -524,9 +541,10 @@ def run_ours(args):
     line = {
         "metric": "48 kHz audio samples/s, encode+quantize+lookup+decode (% HBM roofline in `roofline`)",
         "value": value, "unit": "samples/s", "n_gpus": world, "steps": args.steps, "warmup": args.warmup,
-        "ms_per_step": ms_total / args.steps, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
-        "timed_regions_ms_per_step": [round(r[0] / args.steps, 4) for r in regions],
-        "timed_region_choice": f"median of {len(regions)} back-to-back regions of exactly {args.steps} steps each (barrier + synchronize on both sides of every region)",
+        "ms_per_step": ms_step, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
+        "timed_regions_ms_per_step": [round(r[0], 4) for r in regions], "timed_region_steps": region_steps,
+        "timed_region_choice": f"the {args.steps} timed steps as {len(regions)} back-to-back regions, median region's time per step "
+                               "(barrier + synchronize on both sides of every region)",
         "dtype": "bf16" if args.workload == "v1_bf16" else "f32",
         "data": "synthetic (0.1*randn waveforms, seeded synthetic checkpoint; the reference ships no weights)",
         "config": {"workload": WORKLOAD_NAME[args.workload] + f" batch={B}x{T} per GPU (BASELINE configs[{WORKLOAD_CFG[args.workload]}])",
@@ -752,9 +770,16 @@ def main():
     ap.add_argument("--cpu-utts", type=int, default=192,
                     help="utterances of the bounded CPU sample (192 x 1 s = three steps' worth of audio, 10-15 s of host work)")
     ap.add_argument("--ref-utts", type=int, default=16, help="--impl reference: utterances per step (each step time-bounded at 15 s)")
-    ap.add_argument("--regions", type=int, default=5, help="timed K-step regions measured back to back; the median is reported, all are listed")
+    ap.add_argument("--regions", type=int, default=5,
+                    help="back-to-back regions the K timed steps are split into; the median region is reported, all are listed")
     ap.add_argument("--breakdown", action="store_true", help="print per-launch CUDA-event times to stderr")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's outputs as DIR/waveform.npy (float32) and DIR/indices.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)
